@@ -1,7 +1,8 @@
 #!/usr/bin/env python
-"""Benchmark of the sam_road tiled-inference hot path on B200 (contract: see the task brief / DESIGN.md).
+"""Benchmark of the sam_road tiled-inference hot path on B200 (see DESIGN.md).
 
     python bench.py --gpus 1 --steps 20 --warmup 3                # this framework (CUDA, sm_100a)
+    python bench.py --dump-outputs DIR                            # + the last timed step's results as DIR/*.npy
     python bench.py --workload c4                                 # another BASELINE configuration
     python bench.py --impl reference --steps 3 --warmup 1         # reference algorithm on host CPU cores
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
@@ -72,6 +73,27 @@ SCENE_KEYS = dict(TOPO_THRESHOLD=0.5, ITSC_NMS_RADIUS=8, ROAD_NMS_RADIUS=16, NEI
 
 def flop_per_tile(w):
     return w["flop_tile"] + w["points"] * TOPO_FLOP_PER_POINT
+
+
+DUMP_MAX_VALUES = 4 << 20       # per output (16 MiB of float32): the three outputs stay below 64 MB together
+
+
+def dump_outputs(out_dir, outputs):
+    """Write each result of the last timed step as out_dir/<name>.npy in float32 (None: the workload has
+    no such output).  An output with more than DUMP_MAX_VALUES elements is stored as a fixed sample: the
+    values at seeded random flat indices, in ascending index order, so that two builds run with the same
+    arguments write comparable files."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        if t is None:
+            continue
+        t = t.detach().float()
+        if t.numel() > DUMP_MAX_VALUES:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_MAX_VALUES]
+            t = t.reshape(-1)[idx.sort().values.to(t.device)]
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.cpu().numpy())
 
 
 def load_peaks():
@@ -387,10 +409,10 @@ def run_native(args, w, wl):
                 ex_sc.publish(sl)
                 if NP:
                     ex_ts.publish(sl)
-            return scores, ts
+            return scores, feat, ts
         scores, feat = net.infer_masks_and_img_features(tiles[r])
         ts = net.infer_toponet(feat, *topo[r]) if NP else None
-        return scores, ts
+        return scores, feat, ts
 
     def drain():
         for ex in (ex_sc, ex_ts):
@@ -416,7 +438,8 @@ def run_native(args, w, wl):
         barrier()
         e0.record()
         for i in range(args.steps):
-            step(args.warmup + i)
+            results = None              # a step's results are released before the next step, as in warm-up
+            results = step(args.warmup + i)
         drain()                                            # the last steps' gathers belong to the timed region
         e1.record()
         barrier()
@@ -426,6 +449,10 @@ def run_native(args, w, wl):
     _lib.check(lib.samroad_timing_read(handle, buf, len(buf)), "timing_read")
     kernels = json.loads(buf.value.decode())
     _lib.check(lib.samroad_timing_enable(handle, 0), "timing_disable")
+    if args.dump_outputs and rank == 0:
+        scores, feat, ts = results
+        dump_outputs(args.dump_outputs, dict(mask_scores=scores, image_embeddings=feat, topo_scores=ts))
+    del results
     ms_ranks = [ms]
     if world > 1:
         allms = [torch.zeros(1, device=dev) for _ in range(world)]
@@ -613,7 +640,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--debug-gemm-mode", type=int, default=0,
                     help="A/B only: samroad_debug_disable_2cta_gemm bit mask (16 = no snake traversal)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's mask scores, image embeddings and topology scores to "
+                         "DIR/<name>.npy (float32; outputs above 4 Mi values as a fixed seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs applies to the native arm")
     w = WORKLOADS[args.workload]
     with _JsonStdout() as out:
         _OUT = out
